@@ -199,6 +199,25 @@ int pg_ce_bwd(const void* z, int64_t ld, const int64_t* labels, const float* lse
               int32_t n_rows, int32_t n_total, int32_t c, int dtype, void* g, int64_t ldg, float* colsum,
               float* partial, void* stream);
 
+/*
+ * Multi-label targets (BCEWithLogitsLoss, f1_score(average='micro'): train.py:11-17,317-318) are bit-packed:
+ * ybits is uint32 [rows, lw] with lw >= ceil(c / 32), label j of a row is bit j % 32 of word j / 32, bits >= c are 0.
+ * Logit (and gradient) rows must be 16-byte aligned with ld >= c; any c >= 1 (rows wider than 512 fp32 / 1024 bf16
+ * classes are processed in column chunks of that width).  Outside that: PG_ERR_INVALID.
+ */
+/* loss[0] = sum_{r < n_rows, j < c} max(z, 0) - z * y + log1p(exp(-|z|)), fp32, deterministic;
+ * partial: pg_row_grid(n_rows) * max(c, 1) floats of scratch */
+int pg_bce_fwd(const void* z, int64_t ld, const uint32_t* ybits, int32_t lw, int32_t n_rows, int32_t c, int dtype,
+               float* partial, float* loss, void* stream);
+/* g[r] = (sigmoid(z[r]) - y[r]) * upstream[0] for r < n_rows, 0 for n_rows <= r < n_total; colsum[c] (optional) = the
+ * column sums of g as stored; partial: pg_row_grid(n_total) * c floats */
+int pg_bce_bwd(const void* z, int64_t ld, const uint32_t* ybits, int32_t lw, const float* upstream, int32_t n_rows,
+               int32_t n_total, int32_t c, int dtype, void* g, int64_t ldg, float* colsum, float* partial, void* stream);
+/* counts[0..2] += micro TP, FP, FN of the prediction z > 0 over the rows rows[0..n) (int32 ids into z and ybits; NULL:
+ * rows 0..n); integer adds, deterministic.  The caller zeroes counts. */
+int pg_f1_counts(const void* z, int64_t ld, const uint32_t* ybits, int32_t lw, const int32_t* rows, int32_t n, int32_t c,
+                 int dtype, unsigned long long* counts, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Halo exchange (feature_buffer.py:165-194).  One descriptor per message of a launch; the
  * array lives in device memory and is built once by Buffer.init_buffer.

@@ -75,7 +75,10 @@ def _load():
                                       C.c_int, vp]),
         "pg_ce_fwd": (C.c_int, [vp, i64, vp, i32, i32, C.c_int, vp, vp, vp, vp]),
         "pg_ce_bwd": (C.c_int, [vp, i64, vp, vp, vp, i32, i32, i32, C.c_int, vp, i64, vp, vp, vp]),
-        "pg_push_rows_per_cta": (C.c_int, []),
+        "pg_bce_fwd": (C.c_int, [vp, i64, vp, i32, i32, i32, C.c_int, vp, vp, vp]),
+        "pg_bce_bwd": (C.c_int, [vp, i64, vp, i32, vp, i32, i32, i32, C.c_int, vp, i64, vp, vp, vp]),
+        "pg_f1_counts": (C.c_int, [vp, i64, vp, i32, vp, i32, i32, C.c_int, vp, vp]),
+        "pg_push_rows_per_cta":(C.c_int, []),
         "pg_halo_push": (C.c_int, [vp, i32, i32, vp, i64, i32, C.c_int, f32, f32, u32, vp, vp]),
         "pg_halo_push_drop": (C.c_int, [vp, i32, i32, vp, i64, i32, C.c_int, f32, f32, u32, vp, C.POINTER(pg_drop), vp]),
         "pg_halo_wait": (C.c_int, [vp, i32, u32, vp, i32, vp, vp, vp]),

@@ -701,6 +701,194 @@ ce_bwd2_kernel(const T* __restrict__ z, int64_t ld, const int64_t* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------------------
+// Multi-label (sigmoid) loss and micro-F1 counts over bit-packed 0/1 targets: label j of a row is bit j % 32 of word
+// j / 32 of its lw words.  Same row mapping as the sub-warp cross-entropy kernels (G lanes per row, NVL 16-byte
+// vectors per lane); a vector starts at a multiple of V, which divides 32, so its V label bits sit in one word.
+template <int V>
+__device__ __forceinline__ uint32_t label_bits(const uint32_t* __restrict__ y, int64_t row, int lw, int k0) {
+  return (__ldg(y + row * lw + (k0 >> 5)) >> (k0 & 31)) & ((1u << V) - 1u);
+}
+
+// max(z, 0) - z * y + log1p(exp(-|z|)); the linear part is exact for y in {0, 1}
+__device__ __forceinline__ float bce_term(float z, uint32_t y) {
+  return fmaxf(y ? -z : z, 0.f) + log1pf(expf(-fabsf(z)));
+}
+
+// partial[block] = sum of bce_term over rows < n_rows, columns < c (fixed order: lane, warp, then CTA)
+template <typename T, int G, int NVL>
+__global__ void __launch_bounds__(kRowThreads)
+bce_fwd_kernel(const T* __restrict__ z, int64_t ld, const uint32_t* __restrict__ y, int lw, int n_rows, int c,
+               float* __restrict__ partial) {
+  using P = Pack<T, 16>;
+  using Raw = typename P::Raw;
+  constexpr int V = P::V;
+  constexpr int RPW = 32 / G;
+  __shared__ float wsum[kRowThreads / 32];
+  const int lane = threadIdx.x & 31, lane_g = lane % G, sub = lane / G;
+  const int warp = (blockIdx.x * kRowThreads + threadIdx.x) >> 5;
+  const int warps = (gridDim.x * kRowThreads) >> 5;
+  float acc = 0.f;
+  for (int row0 = warp * RPW; row0 < n_rows; row0 += warps * RPW) {
+    const int row = row0 + sub;
+    if (row >= n_rows) continue;
+    const T* zp = z + static_cast<int64_t>(row) * ld;
+#pragma unroll
+    for (int t = 0; t < NVL; ++t) {
+      const int k0 = (lane_g + t * G) * V;
+      if (k0 >= c) continue;
+      float v[V];
+      P::unpack(*reinterpret_cast<const Raw*>(zp + k0), v);
+      const uint32_t bits = label_bits<V>(y, row, lw, k0);
+#pragma unroll
+      for (int i = 0; i < V; ++i)
+        if (k0 + i < c) acc += bce_term(v[i], (bits >> i) & 1u);
+    }
+  }
+  acc = warp_sum(acc);
+  if (lane == 0) wsum[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float s = 0.f;
+    for (int w = 0; w < kRowThreads / 32; ++w) s += wsum[w];
+    partial[blockIdx.x] = s;
+  }
+}
+
+// g[row, k] = (sigmoid(z) - y) * upstream for row < n_rows, zero for n_rows <= row < n_total; column sums of the stored
+// gradient as in ce_bwd2_kernel (registers, then sub-groups, then the warps of the CTA in fixed order)
+template <typename T, int G, int NVL>
+__global__ void __launch_bounds__(kRowThreads, (NVL * (16 / sizeof(T)) <= 8) ? 4 : (NVL < 4 ? 3 : 2))
+bce_bwd_kernel(const T* __restrict__ z, int64_t ld, const uint32_t* __restrict__ y, int lw,
+               const float* __restrict__ upstream, int n_rows, int n_total, int c, T* __restrict__ g, int64_t ldg,
+               float* __restrict__ partial) {
+  using P = Pack<T, 16>;
+  using Raw = typename P::Raw;
+  constexpr int V = P::V;
+  constexpr int RPW = 32 / G;
+  extern __shared__ float red[];                             // [c]
+  const int lane = threadIdx.x & 31, lane_g = lane % G, sub = lane / G;
+  const int warp = (blockIdx.x * kRowThreads + threadIdx.x) >> 5;
+  const int warps = (gridDim.x * kRowThreads) >> 5;
+  const float up = upstream ? __ldg(upstream) : 1.f;
+  float col[NVL][V];
+#pragma unroll
+  for (int t = 0; t < NVL; ++t)
+#pragma unroll
+    for (int i = 0; i < V; ++i) col[t][i] = 0.f;
+  for (int row0 = warp * RPW; row0 < n_total; row0 += warps * RPW) {
+    const int row = row0 + sub;
+    if (row >= n_total) continue;
+    T* gp = g + static_cast<int64_t>(row) * ldg;
+    const bool train = row < n_rows;
+    const T* zp = z + static_cast<int64_t>(row) * ld;
+#pragma unroll
+    for (int t = 0; t < NVL; ++t) {
+      const int k0 = (lane_g + t * G) * V;
+      if (k0 >= c) continue;
+      float v[V];
+      if (train) {
+        P::unpack(*reinterpret_cast<const Raw*>(zp + k0), v);
+        const uint32_t bits = label_bits<V>(y, row, lw, k0);
+#pragma unroll
+        for (int i = 0; i < V; ++i) v[i] = (1.f / (1.f + expf(-v[i])) - static_cast<float>((bits >> i) & 1u)) * up;
+      } else {
+#pragma unroll
+        for (int i = 0; i < V; ++i) v[i] = 0.f;
+      }
+      const Raw packed = P::pack(v);
+      P::unpack(packed, v);                                    // reduce what is stored
+      if (k0 + V <= c) {
+        st_vec<16>(gp + k0, packed);
+      } else {                                                 // last, partial vector: element stores (exact)
+#pragma unroll
+        for (int i = 0; i < V; ++i)
+          if (k0 + i < c) gp[k0 + i] = static_cast<T>(v[i]);
+      }
+#pragma unroll
+      for (int i = 0; i < V; ++i) col[t][i] += v[i];            // columns >= c are never read out
+    }
+  }
+#pragma unroll
+  for (int t = 0; t < NVL; ++t)
+#pragma unroll
+    for (int i = 0; i < V; ++i)
+#pragma unroll
+      for (int o = G; o < 32; o <<= 1) col[t][i] += __shfl_xor_sync(0xffffffffu, col[t][i], o);
+  for (int i = threadIdx.x; i < c; i += kRowThreads) red[i] = 0.f;
+  __syncthreads();
+  for (int w = 0; w < kRowThreads / 32; ++w) {
+    if ((threadIdx.x >> 5) == w && sub == 0) {
+#pragma unroll
+      for (int t = 0; t < NVL; ++t)
+#pragma unroll
+        for (int i = 0; i < V; ++i) {
+          const int k = (lane_g + t * G) * V + i;
+          if (k < c) red[k] += col[t][i];
+        }
+    }
+    __syncthreads();
+  }
+  float* pp = partial + static_cast<int64_t>(blockIdx.x) * c;
+  for (int i = threadIdx.x; i < c; i += kRowThreads) pp[i] = red[i];
+}
+
+// counts[0..2] += micro TP, FP, FN of the prediction z > 0 over rows rows[0..n) (rows == NULL: 0..n), columns < c.
+// Integer sums: the result does not depend on the order of the adds.
+template <typename T, int G, int NVL>
+__global__ void __launch_bounds__(kRowThreads)
+f1_counts_kernel(const T* __restrict__ z, int64_t ld, const uint32_t* __restrict__ y, int lw,
+                 const int32_t* __restrict__ rows, int n, int c, unsigned long long* __restrict__ counts) {
+  using P = Pack<T, 16>;
+  using Raw = typename P::Raw;
+  constexpr int V = P::V;
+  constexpr int RPW = 32 / G;
+  __shared__ unsigned long long wred[3][kRowThreads / 32];
+  const int lane = threadIdx.x & 31, lane_g = lane % G, sub = lane / G;
+  const int warp = (blockIdx.x * kRowThreads + threadIdx.x) >> 5;
+  const int warps = (gridDim.x * kRowThreads) >> 5;
+  unsigned long long tp = 0, fp = 0, fn = 0;
+  for (int i0 = warp * RPW; i0 < n; i0 += warps * RPW) {
+    const int i = i0 + sub;
+    if (i >= n) continue;
+    const int64_t row = rows ? static_cast<int64_t>(__ldg(rows + i)) : static_cast<int64_t>(i);
+    const T* zp = z + row * ld;
+#pragma unroll
+    for (int t = 0; t < NVL; ++t) {
+      const int k0 = (lane_g + t * G) * V;
+      if (k0 >= c) continue;
+      float v[V];
+      P::unpack(*reinterpret_cast<const Raw*>(zp + k0), v);
+      const uint32_t bits = label_bits<V>(y, row, lw, k0);
+      const uint32_t valid = (k0 + V <= c) ? ((1u << V) - 1u) : ((1u << (c - k0)) - 1u);
+      uint32_t pred = 0;
+#pragma unroll
+      for (int e = 0; e < V; ++e) pred |= (v[e] > 0.f ? 1u : 0u) << e;
+      pred &= valid;
+      tp += __popc(pred & bits);
+      fp += __popc(pred & ~bits);
+      fn += __popc(~pred & bits & valid);
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    tp += __shfl_xor_sync(0xffffffffu, tp, o);
+    fp += __shfl_xor_sync(0xffffffffu, fp, o);
+    fn += __shfl_xor_sync(0xffffffffu, fn, o);
+  }
+  if (lane == 0) {
+    wred[0][threadIdx.x >> 5] = tp;
+    wred[1][threadIdx.x >> 5] = fp;
+    wred[2][threadIdx.x >> 5] = fn;
+  }
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    unsigned long long s = 0;
+    for (int w = 0; w < kRowThreads / 32; ++w) s += wred[threadIdx.x][w];
+    if (s) atomicAdd(counts + threadIdx.x, s);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // Dropout with a counter-based generator: keep(i) is a pure function of (seed, element index), so the backward
 // regenerates the mask instead of storing it.  out = keep ? x / (1 - p) : 0.  16 random bits per element.
 template <typename T>
@@ -899,3 +1087,101 @@ extern "C" int pg_ce_bwd(const void* z, int64_t ld, const int64_t* labels, const
   }
   return PG_OK;
 }
+
+namespace pg {
+// Columns one launch of the multi-label kernels covers: 32 lanes x 4 vectors of 16 bytes (fp32 512, bf16 1024 classes,
+// the row width the cross-entropy kernels keep in registers).  Wider rows are processed in chunks of this many columns,
+// a multiple of 32, so a chunk starts on a label word.
+static int ml_chunk(int es) { return 32 * 4 * (16 / es); }
+
+static const char* ml_check(const void* z, int64_t ld, const uint32_t* ybits, int32_t lw, int32_t c, int dtype) {
+  if (dtype != PG_F32 && dtype != PG_BF16) return "dtype must be PG_F32 or PG_BF16";
+  if (c <= 0) return "c must be >= 1";
+  if (z == nullptr || ybits == nullptr) return "null logits or labels";
+  if (lw < (c + 31) / 32) return "lw must be >= ceil(c / 32)";
+  if (ld < c || vec_bytes(z, ld, elem_size(dtype)) != 16) return "logit rows must be 16-byte aligned with ld >= c";
+  return nullptr;
+}
+}  // namespace pg
+
+#define PG_ML_DISPATCH(KERNEL, T_, NV_, GRID_, SMEM_, ST_, ...) do { \
+    if ((NV_) <= 1) KERNEL<T_, 1, 1><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); \
+    else if ((NV_) <= 2) KERNEL<T_, 2, 1><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); \
+    else if ((NV_) <= 4) KERNEL<T_, 4, 1><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); \
+    else if ((NV_) <= 8) KERNEL<T_, 8, 1><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); \
+    else if ((NV_) <= 16) KERNEL<T_, 16, 1><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); \
+    else if ((NV_) <= 32) KERNEL<T_, 32, 1><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); \
+    else if ((NV_) <= 64) KERNEL<T_, 32, 2><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); \
+    else KERNEL<T_, 32, 4><<<GRID_, kRowThreads, SMEM_, ST_>>>(__VA_ARGS__); } while (0)
+
+extern "C" int pg_bce_fwd(const void* z, int64_t ld, const uint32_t* ybits, int32_t lw, int32_t n_rows, int32_t c,
+                          int dtype, float* partial, float* loss, void* stream) {
+  using namespace pg;
+  const char* bad = ml_check(z, ld, ybits, lw, c, dtype);
+  PG_REQUIRE(bad == nullptr, "pg_bce_fwd: %s (c=%d, lw=%d, ld=%lld)", bad, c, lw, static_cast<long long>(ld));
+  PG_REQUIRE(partial && loss && n_rows >= 0, "pg_bce_fwd: bad argument");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int grid = row_grid(n_rows), es = elem_size(dtype), cw = ml_chunk(es);
+  int n_chunks = 0;
+  for (int c0 = 0; c0 < c; c0 += cw, ++n_chunks) {
+    const int cc = std::min(cw, c - c0), nv = (cc * es + 15) / 16;
+    float* pp = partial + static_cast<int64_t>(n_chunks) * grid;
+    if (dtype == PG_F32)
+      PG_ML_DISPATCH(bce_fwd_kernel, float, nv, grid, 0, st, static_cast<const float*>(z) + c0, ld, ybits + c0 / 32, lw, n_rows, cc, pp);
+    else
+      PG_ML_DISPATCH(bce_fwd_kernel, __nv_bfloat16, nv, grid, 0, st, static_cast<const __nv_bfloat16*>(z) + c0, ld, ybits + c0 / 32, lw, n_rows, cc, pp);
+    PG_LAUNCH_CHECK();
+  }
+  colsum_final_kernel<<<1, 32, 0, st>>>(partial, grid * n_chunks, 1, loss, nullptr, nullptr, 1);
+  PG_LAUNCH_CHECK();
+  return PG_OK;
+}
+
+extern "C" int pg_bce_bwd(const void* z, int64_t ld, const uint32_t* ybits, int32_t lw, const float* upstream,
+                          int32_t n_rows, int32_t n_total, int32_t c, int dtype, void* g, int64_t ldg, float* colsum,
+                          float* partial, void* stream) {
+  using namespace pg;
+  const char* bad = ml_check(z, ld, ybits, lw, c, dtype);
+  PG_REQUIRE(bad == nullptr, "pg_bce_bwd: %s (c=%d, lw=%d, ld=%lld)", bad, c, lw, static_cast<long long>(ld));
+  PG_REQUIRE(g && partial && n_rows >= 0 && n_total >= n_rows, "pg_bce_bwd: bad argument");
+  const int es = elem_size(dtype);
+  PG_REQUIRE(ldg >= c && vec_bytes(g, ldg, es) == 16, "pg_bce_bwd: gradient rows must be 16-byte aligned with ldg >= c");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int grid = row_grid(n_total), cw = ml_chunk(es);
+  for (int c0 = 0; c0 < c; c0 += cw) {
+    const int cc = std::min(cw, c - c0), nv = (cc * es + 15) / 16;
+    const size_t smem = static_cast<size_t>(cc) * sizeof(float);
+    float* pp = partial + static_cast<int64_t>(grid) * c0;
+    if (dtype == PG_F32)
+      PG_ML_DISPATCH(bce_bwd_kernel, float, nv, grid, smem, st, static_cast<const float*>(z) + c0, ld, ybits + c0 / 32, lw, upstream, n_rows, n_total, cc, static_cast<float*>(g) + c0, ldg, pp);
+    else
+      PG_ML_DISPATCH(bce_bwd_kernel, __nv_bfloat16, nv, grid, smem, st, static_cast<const __nv_bfloat16*>(z) + c0, ld, ybits + c0 / 32, lw, upstream, n_rows, n_total, cc, static_cast<__nv_bfloat16*>(g) + c0, ldg, pp);
+    PG_LAUNCH_CHECK();
+    if (colsum != nullptr) {
+      colsum_final_kernel<<<(cc * 32 + 255) / 256, 256, 0, st>>>(pp, grid, cc, colsum + c0, nullptr, nullptr, cc);
+      PG_LAUNCH_CHECK();
+    }
+  }
+  return PG_OK;
+}
+
+extern "C" int pg_f1_counts(const void* z, int64_t ld, const uint32_t* ybits, int32_t lw, const int32_t* rows, int32_t n,
+                            int32_t c, int dtype, unsigned long long* counts, void* stream) {
+  using namespace pg;
+  const char* bad = ml_check(z, ld, ybits, lw, c, dtype);
+  PG_REQUIRE(bad == nullptr, "pg_f1_counts: %s (c=%d, lw=%d, ld=%lld)", bad, c, lw, static_cast<long long>(ld));
+  PG_REQUIRE(counts && n >= 0, "pg_f1_counts: bad argument");
+  if (n == 0) return PG_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int grid = row_grid(n), es = elem_size(dtype), cw = ml_chunk(es);
+  for (int c0 = 0; c0 < c; c0 += cw) {
+    const int cc = std::min(cw, c - c0), nv = (cc * es + 15) / 16;
+    if (dtype == PG_F32)
+      PG_ML_DISPATCH(f1_counts_kernel, float, nv, grid, 0, st, static_cast<const float*>(z) + c0, ld, ybits + c0 / 32, lw, rows, n, cc, counts);
+    else
+      PG_ML_DISPATCH(f1_counts_kernel, __nv_bfloat16, nv, grid, 0, st, static_cast<const __nv_bfloat16*>(z) + c0, ld, ybits + c0 / 32, lw, rows, n, cc, counts);
+    PG_LAUNCH_CHECK();
+  }
+  return PG_OK;
+}
+#undef PG_ML_DISPATCH

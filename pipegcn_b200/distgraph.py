@@ -50,6 +50,9 @@ def _chunked_node_data(n_nodes, n_feat, n_class, mine: torch.Tensor, seed: int, 
 
 def build_rank_layout(spec: dict, rank: int, n_parts: int, device, world=None, seed_graph=0, seed_part=1, seed_feat=2,
                       seed_mask=3, feat_dtype=torch.float32, pair_chunk=32_000_000):
+    if spec.get("multilabel"):
+        raise NotImplementedError("the per-rank graph builder makes single-label graphs only; build multi-label shapes "
+                                  "with synthetic.make_graph")
     dev = torch.device(device)
     n, P, r = int(spec["n_nodes"]), int(n_parts), int(rank)
     i64 = dict(dtype=torch.int64, device=dev)

@@ -29,16 +29,19 @@ def full_graph(g: GlobalGraph, device) -> PartGraph:
 
 
 def calc_acc(logits: torch.Tensor, labels: torch.Tensor) -> float:
-    """train.py:11-17 (multi-label F1 needs sklearn and the yelp dataset: single-label only here)."""
-    if labels.dim() != 1:
-        raise NotImplementedError("multi-label (yelp) evaluation is out of scope")
+    """train.py:11-17: argmax accuracy for [N] labels; for [N, C] 0/1 labels the micro-F1 of `logits > 0`
+    (f1_score(..., average='micro')), counted on the GPU by ops.multilabel_f1."""
+    if labels.dim() == 2:
+        from .ops import multilabel_f1, pack_multilabel
+        return multilabel_f1(logits, pack_multilabel(labels))
     if labels.numel() == 0:
         return float('nan')
     return float((logits.argmax(dim=1) == labels).sum().item()) / labels.shape[0]
 
 
 class EvalSet:
-    """What rank 0 keeps for evaluation: graph(s), features, labels and masks on the device."""
+    """What rank 0 keeps for evaluation: graph(s), features, labels and masks on the device.  Multi-label targets are
+    packed once (`ybits`, ops.pack_multilabel) together with the int32 row ids of every mask (`<mask>_rows`)."""
 
     def __init__(self, g: GlobalGraph, device, inductive: bool = False, dtype=torch.float32):
         self.inductive = bool(inductive)
@@ -46,8 +49,14 @@ class EvalSet:
         val_mask, test_mask = g.val_mask, g.test_mask
 
         def pack(sub: GlobalGraph, masks: Dict[str, torch.Tensor]):
-            return dict(graph=full_graph(sub, dev), feat=sub.feat.to(dev).to(dtype), label=sub.label.to(dev),
-                        **{k: v.to(dev) for k, v in masks.items()})
+            out = dict(graph=full_graph(sub, dev), feat=sub.feat.to(dev).to(dtype), label=sub.label.to(dev),
+                       **{k: v.to(dev) for k, v in masks.items()})
+            if sub.label.dim() == 2:
+                from .ops import pack_multilabel
+                out["ybits"] = pack_multilabel(out.pop("label"))
+                for k in masks:
+                    out[k[:-len("_mask")] + "_rows"] = torch.nonzero(out[k]).flatten().to(torch.int32)
+            return out
 
         if inductive:
             # inductive_split (utils.py): the validation graph holds train+val nodes, the test graph everything
@@ -69,6 +78,15 @@ def _logits(model, part) -> torch.Tensor:
         model.train(was_training)
 
 
+def _score(logits: torch.Tensor, part, mode: str) -> float:
+    """calc_acc over the rows of `<mode>_mask`: accuracy, or micro-F1 against the packed multi-label targets."""
+    if "ybits" in part:
+        from .ops import multilabel_f1
+        return multilabel_f1(logits, part["ybits"], part[mode + "_rows"])
+    mask = part[mode + "_mask"]
+    return calc_acc(logits[mask], part["label"][mask])
+
+
 def _emit(buf: str, result_file_name: Optional[str]):
     if result_file_name is not None:
         os.makedirs(os.path.dirname(result_file_name) or ".", exist_ok=True)
@@ -78,10 +96,11 @@ def _emit(buf: str, result_file_name: Optional[str]):
 
 
 def evaluate_trans(name, model, part, result_file_name=None) -> float:
-    """train.py:42-61: validation and test accuracy on the full graph; returns the validation accuracy."""
+    """train.py:42-61: validation and test accuracy (micro-F1 for a multi-label task, printed as "Accuracy" like the
+    reference) on the full graph; returns the validation score."""
     logits = _logits(model, part)
-    val_acc = calc_acc(logits[part["val_mask"]], part["label"][part["val_mask"]])
-    test_acc = calc_acc(logits[part["test_mask"]], part["label"][part["test_mask"]])
+    val_acc = _score(logits, part, "val")
+    test_acc = _score(logits, part, "test")
     _emit("{:s} | Validation Accuracy {:.2%} | Test Accuracy {:.2%}".format(name, val_acc, test_acc), result_file_name)
     return val_acc
 
@@ -89,8 +108,7 @@ def evaluate_trans(name, model, part, result_file_name=None) -> float:
 def evaluate_induc(name, model, part, mode, result_file_name=None) -> float:
     """train.py:20-39; mode: 'val' or 'test'."""
     logits = _logits(model, part)
-    mask = part[mode + "_mask"]
-    acc = calc_acc(logits[mask], part["label"][mask])
+    acc = _score(logits, part, mode)
     _emit("{:s} | Accuracy {:.2%}".format(name, acc), result_file_name)
     return acc
 
@@ -104,7 +122,8 @@ def result_file(args) -> str:
 
 
 class BestModel:
-    """Best-validation bookkeeping of train.py:377-400: keep the state_dict with the highest validation accuracy,
+    """Best-validation bookkeeping of train.py:377-400: keep the state_dict with the highest validation accuracy
+    (micro-F1 for a multi-label task),
     save it under the reference's key names as `model/<graph_name>_final.pth.tar`."""
 
     def __init__(self):

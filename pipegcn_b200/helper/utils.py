@@ -4,7 +4,7 @@ Counterparts of /root/reference/helper/utils.py: `load_data` (:74-96),
 `graph_partition` (:132-144), `load_partition` (:99-129), `get_layer_size` (:147-151).
 The reference's datasets need DGL, ogb and a network; this engine accepts
 `synthetic:<shape>` datasets (pipegcn_b200/synthetic.py).  The reference's own dataset
-names (`reddit`, `ogbn-products`) are refused unless `PG_ALLOW_SYNTHETIC_FALLBACK=1`
+names (`reddit`, `ogbn-products`, `yelp`) are refused unless `PG_ALLOW_SYNTHETIC_FALLBACK=1`
 is set, in which case the synthetic graph of the same shape (random labels!) is used.
 `get_boundary` (:154-188) has no per-process counterpart: boundary lists come out of
 the one-pass layout builder (pipegcn_b200/partition.py).
@@ -24,7 +24,7 @@ import torch
 from ..partition import PartitionPlan, get_layer_size  # noqa: F401  (re-export)
 from ..synthetic import SHAPES, make_graph, random_partition, train_subgraph
 
-_ALIAS = {'reddit': 'reddit-shaped', 'ogbn-products': 'products-shaped'}
+_ALIAS = {'reddit': 'reddit-shaped', 'ogbn-products': 'products-shaped', 'yelp': 'yelp-shaped'}
 
 
 def _shape_of(dataset: str) -> str:
@@ -43,7 +43,8 @@ def _shape_of(dataset: str) -> str:
 
 
 def load_data(dataset, device='cpu'):
-    """-> (GlobalGraph with one self loop per node, n_feat, n_class)  (utils.py:74-96).  Not cached: the caller
+    """-> (GlobalGraph with one self loop per node, n_feat, n_class)  (utils.py:74-96); for a multi-label shape n_class
+    is the width of the [N, C] label matrix (utils.py:88-91).  Not cached: the caller
     drops the global graph once its partition layout is built."""
     shape = _shape_of(dataset)
     g = make_graph(shape, device=device, planted_labels=os.environ.get('PG_PLANTED_LABELS') == '1')

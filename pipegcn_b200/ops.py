@@ -640,6 +640,106 @@ def cross_entropy_sum(logits, labels, n_train):
     return CrossEntropySum.apply(logits, labels, int(n_train))
 
 
+# ---- multi-label targets (train.py:11-17,317-318): bit-packed on the device ----------------------------------------
+def pack_multilabel(y: torch.Tensor) -> torch.Tensor:
+    """[rows, C] 0/1 labels -> [rows, ceil(C / 32)] 32-bit words; label j is bit j % 32 of word j // 32, bits >= C are
+    0.  The words are held in an int32 tensor (torch's uint32 lacks the copy / add kernels the input pipeline uses);
+    the kernels read them as uint32.  Set-up work (torch ops, any device); the kernels are the only readers."""
+    if y.dim() != 2:
+        raise _C.PgError(f"multi-label targets are [rows, C], got shape {tuple(y.shape)}")
+    rows, c = y.shape
+    lw = (c + 31) // 32
+    bits = torch.zeros(rows, lw * 32, dtype=torch.int64, device=y.device)
+    bits[:, :c] = (y != 0).to(torch.int64)
+    words = (bits.view(rows, lw, 32) << torch.arange(32, device=y.device)).sum(dim=2)
+    return torch.where(words >= 1 << 31, words - (1 << 32), words).to(torch.int32).contiguous()
+
+
+def unpack_multilabel(ybits: torch.Tensor, c: int) -> torch.Tensor:
+    """Inverse of `pack_multilabel`: float32 [rows, c] 0/1."""
+    w = ybits.to(torch.int64) & 0xFFFFFFFF
+    bits = (w.unsqueeze(2) >> torch.arange(32, device=w.device)) & 1
+    return bits.reshape(w.shape[0], -1)[:, :c].to(torch.float32)
+
+
+def _ml_logits(z: torch.Tensor) -> torch.Tensor:
+    """Logits as the multi-label kernels read them: CUDA, fp32/bf16, 16-byte aligned rows (copied only if not)."""
+    _rows(z)
+    if z.dtype not in (torch.float32, torch.bfloat16):
+        z = z.float()
+    return _tma_ready(z)
+
+
+class BceWithLogitsSum(torch.autograd.Function):
+    """BCEWithLogitsLoss(reduction='sum') over the first n_train rows of the logits against bit-packed targets
+    (train.py:317-318); the gradient is zero on the remaining rows (train rows come first after move_train_first)."""
+
+    @staticmethod
+    def forward(ctx, logits, ybits, n_train, c):
+        dev = logits.device
+        n = logits.shape[0]
+        grid = _C.lib.pg_row_grid(max(n_train, 1))
+        partial = torch.empty(grid * max(c, 1), dtype=torch.float32, device=dev)
+        loss = torch.zeros(1, dtype=torch.float32, device=dev)
+        if n_train:
+            _C.count(2)
+            _C.check(_C.lib.pg_bce_fwd(logits.data_ptr(), logits.stride(0), ybits.data_ptr(), ybits.shape[1], n_train,
+                                       c, _C.dtype_code(logits.dtype), partial.data_ptr(), loss.data_ptr(),
+                                       _C.stream_ptr()), "pg_bce_fwd")
+        ctx.save_for_backward(logits, ybits)
+        ctx.n_train, ctx.c, ctx.n = n_train, c, n
+        return loss[0]
+
+    @staticmethod
+    def backward(ctx, up):
+        logits, ybits = ctx.saved_tensors
+        n, c = ctx.n, ctx.c
+        g = alloc_rows(n, c, logits.dtype, logits.device)
+        colsum = torch.empty(c, dtype=torch.float32, device=logits.device)
+        partial = torch.empty(_C.lib.pg_row_grid(n) * c, dtype=torch.float32, device=logits.device)
+        up = up.detach().float().reshape(1).contiguous()
+        _C.count(2)
+        _C.check(_C.lib.pg_bce_bwd(logits.data_ptr(), logits.stride(0), ybits.data_ptr(), ybits.shape[1], up.data_ptr(),
+                                   ctx.n_train, n, c, _C.dtype_code(logits.dtype), g.data_ptr(), g.stride(0),
+                                   colsum.data_ptr(), partial.data_ptr(), _C.stream_ptr()), "pg_bce_bwd")
+        _stash_colsum(g, colsum)
+        return g, None, None, None
+
+
+def bce_with_logits_sum(logits, ybits, n_train, c):
+    """Summed sigmoid cross-entropy of the first n_train rows; `ybits` from `pack_multilabel` (>= n_train rows)."""
+    logits = _ml_logits(logits)
+    assert logits.shape[1] == c and ybits.shape[1] == (c + 31) // 32 and ybits.shape[0] >= n_train
+    return BceWithLogitsSum.apply(logits, ybits, int(n_train), int(c))
+
+
+def f1_counts(logits: torch.Tensor, ybits: torch.Tensor, rows: torch.Tensor = None) -> torch.Tensor:
+    """Device int64 [3] = micro (TP, FP, FN) of `logits > 0` against `ybits` over `rows` (all rows when None)."""
+    z = _ml_logits(logits)
+    n, c = (z.shape[0] if rows is None else int(rows.numel())), z.shape[1]
+    assert ybits.shape[0] == z.shape[0] and ybits.shape[1] == (c + 31) // 32
+    idx = None if rows is None else rows.to(device=z.device, dtype=torch.int32).contiguous()
+    counts = torch.zeros(3, dtype=torch.int64, device=z.device)
+    if n:
+        _C.count()
+        _C.check(_C.lib.pg_f1_counts(z.data_ptr(), z.stride(0), ybits.data_ptr(), ybits.shape[1],
+                                     idx.data_ptr() if idx is not None else None, n, c, _C.dtype_code(z.dtype),
+                                     counts.data_ptr(), _C.stream_ptr()), "pg_f1_counts")
+    return counts
+
+
+def multilabel_f1(logits: torch.Tensor, ybits: torch.Tensor, rows: torch.Tensor = None) -> float:
+    """f1_score(y, logits > 0, average='micro') = 2 TP / (2 TP + FP + FN), one host read.  With no positive label and
+    no positive prediction the score is 0.0, which is what sklearn returns there (zero_division='warn').  A single
+    label column is a binary target to sklearn, whose micro average over the classes {0, 1} is the accuracy."""
+    tp, fp, fn = (int(v) for v in f1_counts(logits, ybits, rows).tolist())
+    if logits.shape[1] == 1:
+        n = logits.shape[0] if rows is None else int(rows.numel())
+        return (n - fp - fn) / n if n else 0.0
+    den = 2 * tp + fp + fn
+    return 2 * tp / den if den else 0.0
+
+
 class Dropout(torch.autograd.Function):
     """Dropout whose mask is regenerated from (seed, element index) in the backward (csrc/rowops.cu)."""
 

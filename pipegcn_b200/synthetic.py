@@ -22,7 +22,7 @@ class GlobalGraph:
     src: torch.Tensor          # [E] int64, message source u
     dst: torch.Tensor          # [E] int64, message destination v (edge u -> v)
     feat: torch.Tensor         # [N, F] float32
-    label: torch.Tensor        # [N] int64
+    label: torch.Tensor        # [N] int64, or [N, C] float32 0/1 for a multi-label shape
     train_mask: torch.Tensor   # [N] bool
 
     @property
@@ -50,7 +50,8 @@ class GlobalGraph:
         return ~self.train_mask & (ids % 2 == 1)
 
 
-# named shapes: nodes, directed edges (incl. self loops), features, classes, train fraction
+# named shapes: nodes, directed edges (incl. self loops), features, classes, train fraction; `multilabel`: every node
+# has a 0/1 vector of n_class labels (BCEWithLogitsLoss + micro-F1, the reference's yelp mode, train.py:11-17,317-318)
 SHAPES = {
     # BASELINE.json configs[1]
     "rmat-1m": dict(n_nodes=1_000_000, n_edges=20_000_000, n_feat=256, n_class=64, train_frac=0.66),
@@ -60,10 +61,22 @@ SHAPES = {
     "products-shaped": dict(n_nodes=2_400_000, n_edges=62_000_000, n_feat=100, n_class=47, train_frac=0.08),
     # configs[4]: built per rank (pipegcn_b200/distgraph.py), never as one global edge list
     "papers100m-shaped": dict(n_nodes=111_000_000, n_edges=1_600_000_000, n_feat=128, n_class=172, train_frac=0.011),
+    # scripts/yelp.sh: Yelp as GraphSAINT ships it -- 716 847 nodes; 13 954 819 directed edges plus one self loop per
+    # node (how the other shapes count edges) = 14 671 666; 300 features; 100 labels per node; 75 % train nodes
+    "yelp-shaped": dict(n_nodes=716_847, n_edges=14_671_666, n_feat=300, n_class=100, train_frac=0.75, multilabel=True),
     # small shapes for tests / smoke
     "tiny": dict(n_nodes=300, n_edges=3_000, n_feat=20, n_class=5, train_frac=0.66),
     "small": dict(n_nodes=20_000, n_edges=400_000, n_feat=64, n_class=16, train_frac=0.66),
+    # multi-label tests: 12 labels (not a multiple of 8 or 32: padded logit rows, a partial label word)
+    "tiny-ml": dict(n_nodes=300, n_edges=3_000, n_feat=20, n_class=12, train_frac=0.66, multilabel=True),
 }
+
+
+def label_rates(n_class: int, seed: int = 5) -> torch.Tensor:
+    """Positive rate p_c of every class of a multi-label shape: log-uniform in [0.01, 0.5], seeded (CPU fp32 [C]).
+    A synthetic choice that gives frequent and rare labels, not Yelp's statistics."""
+    gen = torch.Generator().manual_seed(seed)
+    return torch.exp(torch.empty(n_class).uniform_(math.log(0.01), math.log(0.5), generator=gen))
 
 
 def _rmat_pairs(n_pairs: int, scale: int, gen: torch.Generator, device, abcd=(0.57, 0.19, 0.19, 0.05)):
@@ -121,7 +134,9 @@ def make_graph(shape: str | dict, seed_graph: int = 0, seed_feat: int = 2, seed_
                device="cpu", feat_dtype=torch.float32, planted_labels: bool = False) -> GlobalGraph:
     """Build a named synthetic graph (SURVEY.md §8d seeds: graph 0, features 2, masks 3).
     `planted_labels`: labels = argmax of a fixed random linear map of (own + neighbour-mean) features instead of
-    uniform noise, so that training has something to learn (accuracy tests)."""
+    uniform noise, so that training has something to learn (accuracy tests).  Multi-label shapes: label [N, C] float32
+    0/1, class c positive with rate p_c (`label_rates`); planted, where class c's score under the same kind of map
+    exceeds its (1 - p_c) quantile."""
     spec = SHAPES[shape] if isinstance(shape, str) else dict(shape)
     n = spec["n_nodes"]
     src, dst = rmat_edges(n, spec["n_edges"], seed=seed_graph, device=device)
@@ -129,12 +144,25 @@ def make_graph(shape: str | dict, seed_graph: int = 0, seed_feat: int = 2, seed_
     g = torch.Generator(device=dev)
     g.manual_seed(seed_feat)
     feat = torch.randn(n, spec["n_feat"], generator=g, device=dev, dtype=torch.float32).to(feat_dtype)
-    label = torch.randint(0, spec["n_class"], (n,), generator=g, device=dev)
-    if planted_labels:
+
+    def planted_score():
         proj = torch.randn(spec["n_feat"], spec["n_class"], generator=g, device=dev)
         agg = torch.zeros(n, spec["n_feat"], device=dev).index_add_(0, dst, feat.float()[src])
         agg = agg / torch.bincount(dst, minlength=n).clamp(min=1).unsqueeze(1)
-        label = ((feat.float() + 2.0 * agg) @ proj).argmax(dim=1)
+        return (feat.float() + 2.0 * agg) @ proj
+
+    if spec.get("multilabel"):
+        rate = label_rates(spec["n_class"]).to(dev)
+        if planted_labels:
+            score = planted_score()
+            thr = torch.stack([torch.quantile(score[:, j], 1.0 - rate[j]) for j in range(spec["n_class"])])
+            label = (score > thr).to(torch.float32)
+        else:
+            label = (torch.rand(n, spec["n_class"], generator=g, device=dev) < rate).to(torch.float32)
+    else:
+        label = torch.randint(0, spec["n_class"], (n,), generator=g, device=dev)
+        if planted_labels:
+            label = planted_score().argmax(dim=1)
     g.manual_seed(seed_mask)
     train_mask = torch.rand(n, generator=g, device=dev) < spec["train_frac"]
     if not bool(train_mask.any()):

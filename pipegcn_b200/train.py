@@ -2,7 +2,8 @@
 
 Keeps the entry points of /root/reference/train.py -- `init_processes(rank, size, args)`
 (:408-416) and `run(...)` (:242-400) -- and the order of an epoch (:341-362):
-forward, summed cross-entropy on the local train rows, backward (which runs the
+forward, summed cross-entropy on the local train rows (softmax, or sigmoid for a
+multi-label task, :317-320), backward (which runs the
 gradient halo exchange), `buffer.next_epoch()`, `reducer.synchronize()`, Adam step.
 The DGL partition arguments of the reference's `run(graph, node_dict, gpb, args)` are
 replaced by a `PartitionLayout` (pipegcn_b200/partition.py); evaluation and
@@ -84,7 +85,17 @@ class RankEngine:
         self.part_train = int(tm.sum().item())
         prefix = bool(tm[:self.part_train].all().item()) if self.part_train else True
         self.train_sel = slice(0, self.part_train) if prefix else tm
-        self.labels = layout.label.to(dev)[tm]
+        # multi-label task (the reference's yelp mode, train.py:317-318): [N, C] 0/1 labels, summed sigmoid
+        # cross-entropy; the train rows' labels are kept bit-packed (ops.pack_multilabel)
+        self.multilabel = layout.label.dim() == 2
+        if self.multilabel:
+            from . import ops
+            if not prefix:
+                from ._C import PgError
+                raise PgError("multi-label training needs the train rows first (move_train_first layout)")
+            self.labels = ops.pack_multilabel(layout.label[:self.part_train].to(dev))
+        else:
+            self.labels = layout.label.to(dev)[tm]
         torch.manual_seed(args.seed)                                      # train.py:298
         self.model = create_model(self.layer_size, args, buffer=self.buffer, dtype=self.dtype)
         if init_state is not None:
@@ -170,7 +181,10 @@ class RankEngine:
         self.model.train()
         feat = self.buffer.inner_view(0)
         logits = self.model(self.graph, feat if feat is not None else self.feat, self.in_deg)
-        if isinstance(self.train_sel, slice) and logits.dtype in (torch.float32, torch.bfloat16):
+        if self.multilabel:
+            from . import ops
+            loss = ops.bce_with_logits_sum(logits, self.labels, self.part_train, self.args.n_class)
+        elif isinstance(self.train_sel, slice) and logits.dtype in (torch.float32, torch.bfloat16):
             from . import ops
             loss = ops.cross_entropy_sum(logits, self.labels, self.part_train)      # fused softmax-CE (sum)
         else:
@@ -200,8 +214,9 @@ class RankEngine:
 
     # ---- input pipeline: the next epoch's features travel host -> device while this epoch computes
     def prefetch_features(self, feat_host, label_host=None) -> int:
-        """Start the asynchronous copy of a [N_in, n_feat] pinned host tensor (and optionally the train labels) into one
-        of two staging buffers on a copy stream; returns the slot to hand to `commit_features`."""
+        """Start the asynchronous copy of a [N_in, n_feat] pinned host tensor (and optionally the train labels, in the
+        format of `self.labels`: bit-packed words for a multi-label task) into one of two staging buffers on a copy
+        stream; returns the slot to hand to `commit_features`."""
         if not hasattr(self, '_stage'):
             self._stage_lab = [torch.empty_like(self.labels) for _ in range(2)]
             n_feat = feat_host.shape[1]

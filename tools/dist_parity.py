@@ -31,15 +31,21 @@ def check_mode(world, dev, shape, mode, use_graph, verbose=False):
     """Worst relative error (max over ranks) of this rank's engine against the oracle trace, teacher-forced weights."""
     from oracle.train import initial_state, run_world
     from pipegcn_b200.train import RankEngine
+    from pipegcn_b200.synthetic import SHAPES
     from tests.helpers import make_args, small_world
+    from tests.ml_oracle import multilabel_loss
     rank, size = world.rank, world.size
-    n_class = 5 if shape == "tiny" else 16
+    n_class = SHAPES[shape]["n_class"]
     g, _, layouts, setups = small_world(shape, size)
     n_epochs = 6 if use_graph else 4
     oargs, eargs = make_args(g, n_class, n_epochs=n_epochs, **MODES[mode])
     eargs.cuda_graph = use_graph
     init = initial_state(oargs)
-    traces = run_world(setups, oargs, init_state=init)
+    if g.label.dim() == 2:                                  # multi-label shape: the reference's yelp loss
+        with multilabel_loss():
+            traces = run_world(setups, oargs, init_state=init)
+    else:
+        traces = run_world(setups, oargs, init_state=init)
     eng = RankEngine(layouts[rank], eargs, world, init_state=init, seg_len=32)
     eng.keep_logits = True
     worst = 0.0
